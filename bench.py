@@ -56,7 +56,14 @@ def parse_args():
     ap.add_argument("--skip-train", action="store_true")
     ap.add_argument("--skip-eager", action="store_true")
     ap.add_argument("--skip-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's search result to DIR/D.npy (scores, float32) and "
+                         "DIR/I.npy (ids, float64): every query, or a fixed seeded sample of them beyond 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the result of --impl ours")
     w = WORKLOADS[args.workload]
     args.corpus = args.corpus or w["corpus"]
     args.dim = args.dim or w["dim"]
@@ -346,6 +353,8 @@ def main():
     idx.set_param("profile", 0)
     ms_per_step = total_ms / args.steps
     qps = nq / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, args.dump_outputs, last["D"], last["I"])
 
     e2e_ms = timed(e2e_step, args.steps, min(args.warmup, 2)) / args.steps
     e2e_qps = nq / (e2e_ms * 1e-3)
@@ -469,6 +478,23 @@ def main():
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(torch, out_dir, D, I):
+    """Writes the [nq, k] result of the last timed step as D.npy (float32) and I.npy (int64 ids as float64, exact below
+    2^53).  Rows beyond DUMP_BYTES are dropped by a fixed seeded sample of queries (ascending), so that two builds run
+    with the same arguments, hence the same seeded inputs, can be compared output for output."""
+    import numpy as np
+    nq, k = D.shape
+    fit = (DUMP_BYTES - 4096) // (k * (4 + 8))  # 4096: headroom for the two .npy headers
+    rows = np.arange(nq) if nq <= fit else np.sort(np.random.default_rng(0).choice(nq, fit, replace=False))
+    sel = torch.from_numpy(rows).to(D.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "D.npy"), D[sel].cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "I.npy"), I[sel].cpu().numpy().astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------------------------

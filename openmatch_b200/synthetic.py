@@ -4,8 +4,10 @@ network on the build / GPU boxes).  Weights follow HuggingFace's default initial
 bias paths are exercised); token ids follow SURVEY.md section 8(d)."""
 from __future__ import annotations
 
+import json
 from typing import Dict, Tuple
 
+import numpy as np
 import torch
 
 BERT_BASE = dict(arch="bert", layers=12, hidden=768, heads=12, ffn=3072, vocab=30522, max_pos=512, type_vocab=2,
@@ -63,6 +65,28 @@ def t5_state_dict(spec: Dict, seed: int = 0) -> Dict[str, torch.Tensor]:
         sd[p + "1.DenseReluDense.wi.weight"] = w(F, H, H ** -0.5)
         sd[p + "1.DenseReluDense.wo.weight"] = w(H, F, F ** -0.5)
         sd[p + "1.layer_norm.weight"] = 1.0 + 0.05 * torch.randn(H, generator=g)
+    return sd
+
+
+def _splitmix64(seed: int, n: int) -> np.ndarray:
+    z = np.uint64(seed) + np.arange(1, n + 1, dtype=np.uint64) * np.uint64(0x9E3779B97F4A7C15)
+    z = (z ^ (z >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
+    z = (z ^ (z >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
+    return z ^ (z >> np.uint64(31))
+
+
+def recipe_state_dict(recipe) -> Dict[str, torch.Tensor]:
+    """Weights rebuilt from a recipe: a JSON list (or the list itself) of [name, shape, mean, std, seed] entries, each
+    tensor mean + std * U with U uniform on [-sqrt 3, sqrt 3) at 24-bit resolution, drawn from a splitmix64 stream.
+    Integer arithmetic and correctly rounded float operations only, so the weights are bit-identical on every platform
+    and library version; tests/golden stores such recipes instead of the weights themselves."""
+    if isinstance(recipe, (str, np.ndarray)):
+        recipe = json.loads(str(recipe))
+    sd = {}
+    for name, shape, mean, std, seed in recipe:
+        n = int(np.prod(shape, dtype=np.int64))
+        u = (_splitmix64(seed, n) >> np.uint64(40)).astype(np.int64) - (1 << 23)  # [-2^23, 2^23): exact in float64
+        sd[name] = torch.from_numpy((mean + u * (std * 3.0 ** 0.5 / (1 << 23))).astype(np.float32).reshape(shape))
     return sd
 
 

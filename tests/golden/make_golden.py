@@ -1,9 +1,11 @@
-"""Generates tests/golden/*.npz by executing the REFERENCE's own Python code in the build container:
+"""Generates tests/golden/*.npz by executing the REFERENCE's own Python code (a checkout of thunlp/OpenMatch):
 
-    PYTHONPATH=/root/reference/src python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <path to the OpenMatch checkout>
 
-/root/reference does not exist on the GPU box, so the vectors are committed and this script is only re-run
-here.  What is executed unmodified from the reference:
+The tests do not need the reference, so the vectors are committed.  The models' weights are stored as recipes
+(openmatch_b200.synthetic.recipe_state_dict, with the standard deviations of HF's initialisation) from which the
+tests rebuild them bit for bit; inputs and the reference's outputs are stored as arrays.  What is executed
+unmodified from the reference:
   * openmatch.modeling.DRModelForInference.encode_passage / encode_query  (dense_retrieval_model.py:133-161,261-282)
   * openmatch.loss.SimpleContrastiveLoss                                 (loss.py:7-15)  + torch autograd
   * openmatch.modeling.DRModel.forward (training loss)                    (dense_retrieval_model.py:89-131)
@@ -12,10 +14,12 @@ here.  What is executed unmodified from the reference:
     oracle's FlatIPIndex injected as the `faiss` module (faiss itself is not installable here).
 Models are randomly initialised HF modules (no checkpoints on disk, no network).
 """
+import json
 import os
 import sys
 import tempfile
 import types
+import zlib
 
 import numpy as np
 import torch
@@ -23,14 +27,15 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF_SRC = "/root/reference/src"
-if not os.path.isdir(REF_SRC):
-    sys.exit("reference tree not available; golden vectors can only be regenerated in the build container")
+REF_SRC = os.path.join(os.path.abspath(sys.argv[1]), "src") if len(sys.argv) == 2 else None
+if REF_SRC is None or not os.path.isdir(os.path.join(REF_SRC, "openmatch")):
+    sys.exit("usage: make_golden.py <path to the OpenMatch checkout>")
 sys.path.insert(0, REF_SRC)
 
 import importlib.machinery  # noqa: E402
 
 from oracle.flat_index import FlatIPIndex  # noqa: E402
+from openmatch_b200.synthetic import recipe_state_dict  # noqa: E402
 
 # faiss shim so that `import faiss` in openmatch.retriever succeeds (datasets probes find_spec -> needs __spec__)
 faiss = types.ModuleType("faiss")
@@ -64,8 +69,21 @@ def synth_ids(gen, B, L, vocab, cls_id, sep_id, ragged):
     return ids, mask
 
 
-def sd_to_np(prefix, sd):
-    return {prefix + k: v.detach().cpu().numpy() for k, v in sd.items()}
+def set_recipe_weights(module):
+    """Replaces every floating-point tensor of the module's state dict with zero-mean recipe weights of the tensor's
+    standard deviation (constant tensors keep their value, tied tensors share one seed) and returns the recipe as JSON."""
+    recipe, seeds = [], {}
+    sd = module.state_dict()
+    for name, t in sd.items():
+        if not t.is_floating_point():
+            continue
+        seed = seeds.setdefault(t.data_ptr(), zlib.crc32(name.encode()))
+        std = float("%.4g" % float(t.std())) if t.numel() > 1 else 0.0
+        recipe.append([name, list(t.shape), float(t.flatten()[0]) if std == 0.0 else 0.0, std, seed])
+    with torch.no_grad():
+        for name, w in recipe_state_dict(recipe).items():
+            sd[name].copy_(w)
+    return json.dumps(recipe)
 
 
 def main():
@@ -77,28 +95,29 @@ def main():
     bcfg = BertConfig(vocab_size=512, hidden_size=128, num_hidden_layers=2, num_attention_heads=2,
                       intermediate_size=512, max_position_embeddings=128)
     bert = BertModel(bcfg).eval()
+    bert_recipe = set_recipe_weights(bert)
     margs = ModelArguments(model_name_or_path="unused", pooling="first", normalize=False)
     model = DRModelForInference(lm_q=bert, lm_p=bert, tied=True, pooling="first", normalize=False, model_args=margs)
     ids, mask = synth_ids(gen, 6, 32, 512, 101, 102, ragged=True)
     tt = torch.zeros_like(ids)
     hidden, reps = model.encode_passage({"input_ids": ids, "attention_mask": mask, "token_type_ids": tt})
     np.savez_compressed(os.path.join(HERE, "bert_small.npz"), input_ids=ids.numpy(), attention_mask=mask.numpy(),
-                        token_type_ids=tt.numpy(), hidden=hidden.numpy(), reps=reps.numpy(),
-                        **sd_to_np("sd.", bert.state_dict()))
+                        token_type_ids=tt.numpy(), hidden=hidden.numpy(), reps=reps.numpy(), sd_recipe=bert_recipe)
 
     # ---------------- T5 encoder, mean pooling + linear head + normalise (GTR-style) ----------------
     tcfg = T5Config(vocab_size=512, d_model=128, d_kv=64, d_ff=512, num_layers=2, num_heads=2,
                     feed_forward_proj="relu")
     t5 = T5EncoderModel(tcfg).eval()
+    t5_recipe = set_recipe_weights(t5)
     head = LinearHead(128, 128)
+    head_recipe = set_recipe_weights(head)  # one entry: "linear.weight"
     margs = ModelArguments(model_name_or_path="unused", pooling="mean", normalize=True, encoder_only=True)
     model = DRModelForInference(lm_q=t5, lm_p=t5, tied=True, pooling="mean", normalize=True, head_q=head, head_p=head,
                                 model_args=margs)
     ids, mask = synth_ids(gen, 6, 32, 512, None, 1, ragged=True)
     hidden, reps = model.encode_passage({"input_ids": ids, "attention_mask": mask})
     np.savez_compressed(os.path.join(HERE, "t5_small.npz"), input_ids=ids.numpy(), attention_mask=mask.numpy(),
-                        hidden=hidden.numpy(), reps=reps.numpy(), head_weight=head.linear.weight.detach().numpy(),
-                        **sd_to_np("sd.", t5.state_dict()))
+                        hidden=hidden.numpy(), reps=reps.numpy(), sd_recipe=t5_recipe, head_recipe=head_recipe)
 
     # ---------------- T5 relative-position buckets for every distance the encoder can see ----------------
     from transformers.models.t5.modeling_t5 import T5Attention

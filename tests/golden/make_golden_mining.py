@@ -1,6 +1,6 @@
-"""Generates tests/golden/mining.json by executing the REFERENCE's own hard-negative selection in the build container:
+"""Generates tests/golden/mining.json by executing the REFERENCE's own hard-negative selection:
 
-    python tests/golden/make_golden_mining.py
+    python tests/golden/make_golden_mining.py <path to the OpenMatch checkout>
 
 scripts/msmarco/build_hn.py is a script (argparse runs at import), so the generator lifts only the source of its
 ``load_ranking`` function out of the file with ``ast`` and executes it unmodified against a synthetic TREC run with
@@ -13,9 +13,9 @@ import random
 import sys
 import tempfile
 
-REF = "/root/reference/scripts/msmarco/build_hn.py"
-if not os.path.exists(REF):
-    sys.exit("reference tree not available; golden vectors can only be regenerated in the build container")
+REF = os.path.join(sys.argv[1], "scripts", "msmarco", "build_hn.py") if len(sys.argv) == 2 else None
+if REF is None or not os.path.exists(REF):
+    sys.exit("usage: make_golden_mining.py <path to the OpenMatch checkout>")
 src = open(REF).read()
 fn = next(n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name == "load_ranking")
 ns = {"random": random}

@@ -2,7 +2,7 @@
 (encoder_only=False: full encoder-decoder, one zero decoder token, reps = decoder last_hidden_state[:, 0];
 src/openmatch/modeling/dense_retrieval_model.py:137-141) on a randomly initialised tiny T5Model:
 
-    PYTHONPATH=/root/reference/src python tests/golden/make_golden_t5dec.py
+    python tests/golden/make_golden_t5dec.py <path to the OpenMatch checkout>
 """
 import os
 import sys
@@ -10,9 +10,9 @@ import sys
 import numpy as np
 import torch
 
-REF_SRC = "/root/reference/src"
-if not os.path.isdir(REF_SRC):
-    sys.exit("reference tree not available; golden vectors can only be regenerated in the build container")
+REF_SRC = os.path.join(os.path.abspath(sys.argv[1]), "src") if len(sys.argv) == 2 else None
+if REF_SRC is None or not os.path.isdir(os.path.join(REF_SRC, "openmatch")):
+    sys.exit("usage: make_golden_t5dec.py <path to the OpenMatch checkout>")
 sys.path.insert(0, REF_SRC)
 from transformers import T5Config, T5Model  # noqa: E402
 

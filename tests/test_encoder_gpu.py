@@ -11,6 +11,7 @@ import pytest
 import torch
 
 import oracle
+from openmatch_b200.synthetic import recipe_state_dict
 from oracle.encoder import EncoderSpec
 
 pytestmark = pytest.mark.gpu
@@ -38,8 +39,7 @@ def _check(got, want, what, rel_tol=1e-2, cos_tol=0.9999):
 
 def _golden(golden_dir, name):
     z = np.load(os.path.join(golden_dir, name))
-    sd = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd.")}
-    return z, sd
+    return z, recipe_state_dict(z["sd_recipe"])
 
 
 def test_bert_small_matches_reference_golden(enc_mod, golden_dir):
@@ -59,8 +59,8 @@ def test_t5_small_matches_reference_golden(enc_mod, golden_dir):
     z, sd = _golden(golden_dir, "t5_small.npz")
     spec = dict(arch="t5", layers=2, hidden=128, heads=2, ffn=512, vocab=512, ln_eps=1e-6, rel_buckets=32,
                 rel_max_distance=128)
-    enc = enc_mod.CudaEncoder(spec, sd, head_weight=torch.from_numpy(z["head_weight"]), pooling="mean", normalize=True,
-                              max_batch_tokens=1024)
+    head_w = recipe_state_dict(z["head_recipe"])["linear.weight"]
+    enc = enc_mod.CudaEncoder(spec, sd, head_weight=head_w, pooling="mean", normalize=True, max_batch_tokens=1024)
     ids, mask = (torch.from_numpy(z[k]).cuda() for k in ("input_ids", "attention_mask"))
     hidden, reps = enc.encode(ids, mask, return_hidden=True)
     m = z["attention_mask"].astype(bool)

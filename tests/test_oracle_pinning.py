@@ -1,18 +1,18 @@
 """CPU: pins the oracle (oracle/*.py) against golden vectors produced by the REFERENCE's own code
-(tests/golden/make_golden.py, executed in the build container against /root/reference/src/openmatch)."""
+(tests/golden/make_golden.py, executed against a checkout of thunlp/OpenMatch)."""
 import os
 
 import numpy as np
 import torch
 
 import oracle
+from openmatch_b200.synthetic import recipe_state_dict
 from oracle.encoder import EncoderSpec
 
 
 def _load(golden_dir, name):
     z = np.load(os.path.join(golden_dir, name), allow_pickle=False)
-    sd = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd.")}
-    return z, sd
+    return z, recipe_state_dict(z["sd_recipe"])
 
 
 def test_bert_encoder_matches_reference(golden_dir):
@@ -30,7 +30,7 @@ def test_t5_encoder_matches_reference(golden_dir):
     z, sd = _load(golden_dir, "t5_small.npz")
     spec = EncoderSpec("t5", layers=2, hidden=128, heads=2, ffn=512, ln_eps=1e-6, pooling="mean", normalize=True)
     hidden, reps = oracle.encode_reps(sd, spec, torch.from_numpy(z["input_ids"]), torch.from_numpy(z["attention_mask"]),
-                                      head_weight=torch.from_numpy(z["head_weight"]))
+                                      head_weight=recipe_state_dict(z["head_recipe"])["linear.weight"])
     m = z["attention_mask"].astype(bool)
     np.testing.assert_allclose(hidden.numpy()[m], z["hidden"][m], rtol=2e-4, atol=2e-5)
     np.testing.assert_allclose(reps.numpy(), z["reps"], rtol=2e-4, atol=2e-6)

@@ -29,11 +29,13 @@ def small_bert(golden_dir):
     if not torch.cuda.is_available():
         pytest.skip("needs a CUDA device")
     from transformers import BertConfig, BertModel
+
+    from openmatch_b200.synthetic import recipe_state_dict
     z = np.load(os.path.join(golden_dir, "bert_small.npz"))
     cfg = BertConfig(vocab_size=512, hidden_size=128, num_hidden_layers=2, num_attention_heads=2, intermediate_size=512,
                      max_position_embeddings=128)
     lm = BertModel(cfg)
-    sd = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd.")}
+    sd = recipe_state_dict(z["sd_recipe"])
     missing, unexpected = lm.load_state_dict(sd, strict=False)
     assert not [m for m in missing if "position_ids" not in m], missing
     return lm.eval()
